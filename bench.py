@@ -25,6 +25,7 @@ sys.path.insert(0, ROOT)
 FLOP_PER_FRAME = 85_710_602_240          # ROMP HRNet-32 + heads @512x512 (SURVEY 8d, hooked on the reference)
 SMPL_BYTES_PER_PERSON = 83_860
 BATCH = 64
+DUMP_LIMIT_BYTES = 63_000_000           # --dump-outputs stays under 64 MB, .npy headers included
 
 
 def measured_peaks():
@@ -125,6 +126,33 @@ def run_reference(args):
 def _events():
     import torch
     return torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+
+
+def dump_outputs(path, arrays):
+    """Write the result arrays of the last timed step as path/<name>.npy so that two builds can be compared output for
+    output: integer arrays as float64 (exact), the rest as float32.  ``arrays`` maps names to numpy arrays or device
+    tensors that all index persons along their first axis.  Above DUMP_LIMIT_BYTES in all, every array keeps the same
+    rows: a seeded sample of the persons, in ascending order, taken on the device before the read-back."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    if not arrays:
+        return
+    dtypes = {}
+    for name, v in arrays.items():
+        dt = (v[:0].cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v)).dtype
+        dtypes[name] = np.dtype(np.float64 if dt == np.float64 or dt.kind in "iub" else np.float32)
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(int(np.prod(v.shape[1:])) * dtypes[name].itemsize for name, v in arrays.items())
+    rows = None
+    if n * row_bytes > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT_BYTES // row_bytes, replace=False))
+    for name, v in arrays.items():
+        dt = dtypes[name]
+        if rows is not None:
+            v = v[torch.from_numpy(rows).to(v.device)] if isinstance(v, torch.Tensor) else v[rows]
+        if isinstance(v, torch.Tensor):
+            v = v.cpu().numpy()
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(v, dtype=dt))
 
 
 def committed_traffic(precision):
@@ -283,6 +311,8 @@ def run_ours(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)     # rank 0's shard of the last end-to-end step
     fps = world * B * steps / t_dev
     net_tflops = B * steps * FLOP_PER_FRAME / t_net / 1e12          # per GPU
     nb, _ = model._net(2)
@@ -390,6 +420,8 @@ def run_smpl(args, emit_line=True):
     e1.record(st)
     st.synchronize()
     ms = e0.elapsed_time(e1) / steps
+    if emit_line and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"verts": verts, "joints": joints})
     peaks = measured_peaks()
     gbs = n * SMPL_BYTES_PER_PERSON / ms / 1e6
     res = {
@@ -445,6 +477,8 @@ def run_bev(args, emit_line=True):
         out = m.forward_batch(frames_host, center3d_override=vol)
     torch.cuda.synchronize()
     t_e2e = time.perf_counter() - w0
+    if emit_line and args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     peaks = measured_peaks()
     fps = B * steps / t_dev
     res = {
@@ -480,7 +514,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", dest="no_cpu_baseline", action="store_true")
     ap.add_argument("--no-extra", dest="no_extra", action="store_true",
                     help="skip the extra legs of the N=1 line (sustained window, TF32 engine, cfg3/cfg5, PyTorch-CUDA comparator)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="after the timed steps, write the results of the last one as DIR/<name>.npy (float32 / float64, "
+                         "at most 64 MB: a seeded sample of the persons when the whole is larger)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours")
     # stdout carries exactly ONE line (the JSON): library chatter written to file descriptor 1 while we run (NCCL prints
     # its version banner there on the first communicator) is diverted to stderr; emit() restores the real stdout.
     global _REAL_STDOUT
