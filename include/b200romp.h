@@ -236,6 +236,37 @@ int b200romp_bev_post(const float* betas, const float* verts_smil, const float* 
 /* dst[i] = src[sel[i]] for i < *d_count; rows of row_bytes (multiple of 4) bytes. */
 int b200romp_gather_rows(const void* src, int row_bytes, const int* sel, const int* d_count, int capacity, void* dst,
                          b200romp_stream stream);
+/* the same with dst row offset *d_base (device int32): dst[*d_base + i] = src[sel[i]] - appends rows without a host sync */
+int b200romp_gather_rows_at(const void* src, int row_bytes, const int* sel, const int* d_count, const int* d_base, int capacity,
+                            void* dst, b200romp_stream stream);
+
+/* BEV crowd mode, BEV.process_long_image (bev/main.py:184-258, bev/split2process.py) for images with w/h >= 2.
+ * plan = DEVICE int32 [n_crops][2]: crop c covers rows 0..h-1 and columns [plan[c][0], plan[c][1]) of the image padded by
+ * `pad` zero columns on each side (padding_image_overlap / get_image_split_plan, split2process.py:6-39; the last crop is
+ * narrower than h).
+ *
+ * Per chunk of crops first_crop .. first_crop+batch-1 whose detections (batch_ids = crop - first_crop) went through
+ * b200romp_bev_regress and SMPL-A / SMIL:  SMIL baby merge (post_parser.py:255-278); exclude_boudary_subjects
+ * (split2process.py:41-46) on every crop but the last (cam_x > 1 - r_c, main.py:209-215) and on crops 2..S-1
+ * (cam_x < r_{c-1} - 1, :221-226; crop 1 is never tested); projection in crop pixels (offsets [0,h,0,cw,h,cw], :216-218);
+ * per crop suppressing_redundant_prediction_via_projection(conf_based=True) and remove_outlier(scale_thresh=1) (:228-232)
+ * with crop_nms_thr_px = nms_thresh * h / 640 (fp32); convert_crop_cam_params2full_image (split2process.py:48-58, :242-248)
+ * into cam_full [cap,3].  The survivors' indices go to sel / *d_count_sel in order, *d_base receives the device counter
+ * *d_merged, which advances by their number (at most merged_capacity): append them with b200romp_gather_rows_at.
+ * flags: int32 [2*capacity] scratch. */
+int b200romp_bev_long_crops(const float* betas, const float* verts_smil, const float* joints_smil, float* verts, float* joints,
+                            const float* cam, const float* cam_trans, const float* conf, const long long* batch_ids, int batch,
+                            int capacity, const int* d_count, const int* plan, int n_crops, int first_crop, int h, int w, int pad,
+                            float crop_nms_thr_px, float rel_scale_thresh, float* pj2d_org, float* cam_full, int* flags, int* sel,
+                            int* d_count_sel, int* d_base, int* d_merged, int merged_capacity, b200romp_stream stream);
+/* The final stage over the *d_count merged people (main.py:253-256): cam_trans from the full-image cams
+ * (denormalize_cam_params_to_trans), projection with image_pad_info [(w-h)/2, ., 0, w, h, w] (split2process.py:16-21),
+ * suppressing_redundant_prediction_via_projection(conf_based=True) with nms_thr_px = nms_thresh * max(h, w) / 640 (fp32)
+ * over all pairs at once, then remove_outlier(scale_thresh=0.5).  Survivors -> sel / *d_count_out in order.
+ * workspace: int32 [3*capacity + 1]; capacity <= 65535. */
+int b200romp_bev_long_merge(const float* joints, const float* cam, const float* conf, int capacity, const int* d_count, int h, int w,
+                            float nms_thr_px, float rel_scale_thresh, float* cam_trans, float* pj2d_org, int* workspace, int* sel,
+                            int* d_count_out, b200romp_stream stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Row a1/f2: `img_preprocess(image)` (simple_romp/romp/utils.py:16-30, called from ROMP.forward main.py:161): BGR->RGB,
@@ -245,6 +276,13 @@ int b200romp_gather_rows(const void* src, int row_bytes, const int* sel, const i
  * pad_info6 (HOST, may be NULL) receives [top, bottom, left, right, h, w] like padding_image. */
 int b200romp_preprocess_bgr(const unsigned char* img_bgr_device, int h, int w, int row_stride_bytes, int out_size,
                             unsigned char* out_rgb_device, float* pad_info6_host, b200romp_stream stream);
+/* BEV crowd mode (bev/main.py:193-199): img_preprocess of crops first_crop .. first_crop+n_crops-1 of the padded wide
+ * image in one launch, without materialising the padding: columns outside the unpadded image (pad zero columns on each
+ * side, split2process.py:6-13) and the centre padding of a crop narrower than h read as zero.  plan = DEVICE int32
+ * [.][2] as for b200romp_bev_long_crops.  out_rgb [n_crops, out_size, out_size, 3]; bit-exact like b200romp_preprocess_bgr. */
+int b200romp_preprocess_crops_bgr(const unsigned char* img_bgr_device, int h, int w, int row_stride_bytes, int pad,
+                                  const int* plan_device, int first_crop, int n_crops, int out_size, unsigned char* out_rgb_device,
+                                  b200romp_stream stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Row f4: the temporal stage of ROMP.forward with --temporal_optimize (main.py:117-157): One-Euro smoothing of

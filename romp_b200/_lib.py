@@ -154,11 +154,16 @@ def load():
     _sig(lib.b200romp_bev_regress, i32, vp, vp, vp, i32, vp, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp)
     _sig(lib.b200romp_bev_post, i32, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, vp, fp, f32, f32, f32, vp, vp, vp, vp, vp)
     _sig(lib.b200romp_gather_rows, i32, vp, i32, vp, vp, i32, vp, vp)
+    _sig(lib.b200romp_gather_rows_at, i32, vp, i32, vp, vp, vp, i32, vp, vp)
+    _sig(lib.b200romp_bev_long_crops, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, vp, vp, i32, i32, i32, i32, i32, f32, f32,
+         vp, vp, vp, vp, vp, vp, vp, i32, vp)
+    _sig(lib.b200romp_bev_long_merge, i32, vp, vp, vp, i32, vp, i32, i32, f32, f32, vp, vp, vp, vp, vp, vp)
     _sig(lib.b200romp_tracks_create, vp, i32, i32)
     _sig(lib.b200romp_tracks_destroy, None, vp)
     _sig(lib.b200romp_tracks_reset, i32, vp, i32, vp)
     _sig(lib.b200romp_one_euro_smooth, i32, vp, vp, i32, vp, vp, vp, i32, i32, vp, f32, f32, vp)
     _sig(lib.b200romp_preprocess_bgr, i32, vp, i32, i32, i32, i32, vp, fp, vp)
+    _sig(lib.b200romp_preprocess_crops_bgr, i32, vp, i32, i32, i32, i32, vp, i32, i32, i32, vp, vp)
     _sig(lib.b200romp_pack_rows, i32, C.POINTER(vp), ip, i32, vp, i32, i32, i32, i32, vp, i32, vp)
     if lib.b200romp_version() != 200:
         raise RuntimeError("libb200romp.so version mismatch - rebuild")
@@ -185,5 +190,6 @@ EXPORTS = [
     "b200romp_bev_create", "b200romp_bev_destroy", "b200romp_bev_bv_input", "b200romp_bev_center3d",
     "b200romp_bev_parse_workspace_bytes", "b200romp_bev_parse3d", "b200romp_bev_regress", "b200romp_bev_post",
     "b200romp_gather_rows", "b200romp_pack_rows", "b200romp_preprocess_bgr", "b200romp_tracks_create", "b200romp_tracks_destroy",
-    "b200romp_tracks_reset", "b200romp_one_euro_smooth",
+    "b200romp_tracks_reset", "b200romp_one_euro_smooth", "b200romp_gather_rows_at", "b200romp_bev_long_crops",
+    "b200romp_bev_long_merge", "b200romp_preprocess_crops_bgr",
 ]

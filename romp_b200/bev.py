@@ -2,7 +2,8 @@
 
 ``bev_settings`` mirrors bev/main.py:27-87 (same flags and defaults, including the quirk that ``crowd`` defaults to
 True and therefore overrides the thresholds with ``long_conf_dict``), ``BEV(settings)(image_bgr) -> dict | None``
-mirrors bev/main.py:91-181 for normal (non-panoramic) images; ``forward_batch`` is the batched entry point.
+mirrors bev/main.py:91-181: normal images, and with ``crowd`` images of aspect ratio >= 2 through the sliding-window
+``process_long_image`` (bev/main.py:184-258); ``forward_batch`` is the batched entry point.
 Per-frame semantics of the two post filters (bev/post_parser.py:167-222) are preserved by applying them per
 ``pred_batch_ids`` group on the device.  Python only allocates buffers and sequences library calls.
 """
@@ -68,6 +69,23 @@ def bev_settings(input_args=sys.argv[1:]):
         args.center_thresh, args.nms_thresh = long_conf_dict[args.model_id][0], long_conf_dict[args.model_id][1]
         args.relative_scale_thresh, args.overlap_ratio = long_conf_dict[model_id][2], long_conf_dict[args.model_id][3]
     return args
+
+
+def long_image_plan(h, w, overlap):
+    """padding_image_overlap + get_image_split_plan (bev/split2process.py:6-39) -> (int32 [S,2] crop columns [left, right)
+    of the image padded by ``pad`` zero columns on each side, pad).  Every crop spans the full height h; the last one
+    starts at W-h but keeps the right edge of crop S-2 (:33-37), so it is narrower than h."""
+    pad = int(h * overlap)
+    W = w + 2 * pad
+    S = int(np.ceil((W / h - 1) / (1 - overlap))) + 1
+    step = (1 - overlap) * h
+    boxes, right = [], None
+    for i in range(S):
+        left = W - h if i == S - 1 else step * i
+        if i != S - 1:
+            right = left + h
+        boxes.append([left, right])
+    return np.array(boxes).astype(np.int32), pad
 
 
 class BEV(torch.nn.Module):
@@ -242,11 +260,148 @@ class BEV(torch.nn.Module):
             self.run_post(B, offsets if offsets is not None else [0, 512, 0, 512, 512, 512], img_max_side)
         return self.collect(to_numpy)
 
+    # ------------------------------------------------------------------------------------------
+    _long_fields = ("thetas", "betas", "cam", "params_pred", "conf", "verts", "joints")
+
+    def _long_alloc(self, mcap):
+        """Merged buffers of crowd mode for up to ``mcap`` people (S crops x 64), grown on demand."""
+        if getattr(self, "_long", None) is not None and self._long["mcap"] >= mcap:
+            return self._long
+        self._long = None
+        dev, b = self.tdevice, self.buf
+        z = lambda *shape, dtype=torch.float32: torch.zeros(*shape, dtype=dtype, device=dev)
+        L = {"mcap": mcap, "cam_full": z(self.cap, 3), "flags": z(2 * self.cap, dtype=torch.int32), "base": z(1, dtype=torch.int32),
+             "merged": z(1, dtype=torch.int32), "cam_trans": z(mcap, 3), "pj2d_org": z(mcap, 71, 2),
+             "ws": z(3 * mcap + 1, dtype=torch.int32), "sel": z(mcap, dtype=torch.int32), "count_out": z(1, dtype=torch.int32),
+             "plan": z(2 * mcap, dtype=torch.int32), "plan_host": torch.zeros(2 * mcap, dtype=torch.int32).pin_memory()}
+        L["m"] = {k: z(mcap, *b[k].shape[1:]) for k in self._long_fields}
+        L["o"] = {k: z(mcap, *b[k].shape[1:]) for k in self._long_fields + ("cam_trans", "pj2d_org")}
+        self._long = L
+        return L
+
+    def _long_upload(self, img):
+        """raw HxWx3 uint8 image -> device, on self.stream, without a host sync: a host image goes through a pinned buffer
+        (free again: every call ends with the stream synchronised by ``collect``)."""
+        if img.is_cuda:
+            cur = torch.cuda.current_stream(self.tdevice)
+            if cur != self.stream:
+                self.stream.wait_stream(cur)
+            img.record_stream(self.stream)
+            return img.contiguous()
+        n = img.numel()
+        if getattr(self, "_raw_host", None) is None or self._raw_host.numel() < n:
+            self._raw_host = torch.empty(max(n, 1 << 22), dtype=torch.uint8).pin_memory()
+            self._raw_dev = torch.empty(self._raw_host.numel(), dtype=torch.uint8, device=self.tdevice)
+        self._raw_host[:n].copy_(img.reshape(-1))
+        raw = self._raw_dev[:n]
+        raw.copy_(self._raw_host[:n], non_blocking=True)
+        return raw
+
+    @torch.no_grad()
+    def process_long_image(self, full_image, show_patch_results=False, center3d_override=None, to_numpy=True):
+        """BEV.process_long_image (bev/main.py:184-258): crowd mode for images with w/h >= 2.  The image is padded by
+        int(h * overlap_ratio) zero columns on each side and cut into S overlapping full-height crops
+        (bev/split2process.py); the crops run as batches of <= max_batch through the batched BEV path, every per-crop
+        and merge step runs on the device, and the only host synchronisation is the final person count.
+
+        full_image: HxWx3 uint8 BGR, numpy or tensor (host or device).  center3d_override [S,64,128,128] replaces each
+        crop's 3-D centre map (tests).  Returns the dict of ``forward_batch`` (pred_batch_ids all 0, full-image cam /
+        cam_trans / pj2d_org) or None.  Deliberate differences to the reference: a crop without detections contributes
+        nothing (the reference's crop bookkeeping misaligns and raises), and an image without survivors returns None
+        (the reference raises KeyError)."""
+        if show_patch_results:
+            raise NotImplementedError("show_patch_results renders every crop; rendering is outside the B200 hot path")
+        if not self.calc_smpl:
+            raise ValueError("crowd mode (images with w/h >= 2 and --crowd on) needs SMPL: the crops are merged on projected "
+                             "joints, so build BEV with calc_smpl on")
+        img = torch.from_numpy(np.ascontiguousarray(full_image)) if isinstance(full_image, np.ndarray) else full_image
+        assert img.dtype == torch.uint8 and img.dim() == 3 and img.shape[2] == 3, "image must be HxWx3 uint8 (BGR)"
+        h, w = int(img.shape[0]), int(img.shape[1])
+        plan, pad = long_image_plan(h, w, float(self.settings.overlap_ratio))
+        S = len(plan)
+        assert S >= 2 and int((plan[:, 1] - plan[:, 0]).max()) <= h, "crowd mode needs w/h >= 2"
+        L = self._long_alloc(S * MAX_PERSON)
+        if center3d_override is not None:
+            center3d_override = torch.as_tensor(center3d_override, dtype=torch.float32, device=self.tdevice)
+            assert tuple(center3d_override.shape) == (S, 64, 128, 128), "center3d_override must be [S,64,128,128]"
+        cur = torch.cuda.current_stream(self.tdevice)
+        if center3d_override is not None and cur != self.stream:
+            self.stream.wait_stream(cur)
+        with torch.cuda.stream(self.stream):
+            raw = self._long_upload(img)
+            self._long_begin(plan)
+            for c0 in range(0, S, self.max_batch):
+                nb = min(self.max_batch, S - c0)
+                key = (torch.uint8, nb)
+                if key not in self._staging:
+                    self._staging[key] = torch.empty((nb, 512, 512, 3), dtype=torch.uint8, device=self.tdevice)
+                fd = self._staging[key]
+                _lib.check(self.lib.b200romp_preprocess_crops_bgr(_ptr(raw), h, w, 3 * w, pad, _ptr(L["plan"]), c0, nb, 512, _ptr(fd),
+                                                                  C.c_void_p(self.stream.cuda_stream)), "preprocess_crops_bgr")
+                self.run_model(fd, None if center3d_override is None else center3d_override[c0:c0 + nb])
+                self._long_chunk(plan, pad, c0, nb, h, w)
+            self._long_finish(h, w)
+        return self._long_collect(to_numpy)
+
+    def _long_begin(self, plan):
+        L = self._long
+        L["plan_host"][:plan.size].copy_(torch.from_numpy(plan.reshape(-1)))
+        L["plan"][:plan.size].copy_(L["plan_host"][:plan.size], non_blocking=True)
+        L["merged"].zero_()
+
+    def _long_chunk(self, plan, pad, c0, nb, h, w):
+        """Crops c0 .. c0+nb-1, detected and regressed into self.buf (batch_ids = crop - c0): SMPL-A / SMIL, then
+        bev/main.py:203-249 on the device, survivors appended to the merged buffers."""
+        lib, b, L, sp, ck = self.lib, self.buf, self._long, C.c_void_p(self.stream.cuda_stream), _lib.check
+        s, st = self.settings, self.stream.cuda_stream
+        self.smpla.forward(b["betas"], b["thetas"], self.cap, b["count"], True, b["smpl_ws"], b["verts"], b["joints"], st)
+        self.smil.forward(b["betas"], b["thetas"], self.cap, b["count"], True, b["smpl_ws"], b["verts_smil"], b["joints_smil"], st)
+        crop_thr = float(s.nms_thresh) * h / 640          # nms_thresh * max(crop h, crop w) / 640 (post_parser.py:186-187)
+        ck(lib.b200romp_bev_long_crops(_ptr(b["betas"]), _ptr(b["verts_smil"]), _ptr(b["joints_smil"]), _ptr(b["verts"]),
+                                       _ptr(b["joints"]), _ptr(b["cam"]), _ptr(b["cam_trans"]), _ptr(b["conf"]), _ptr(b["batch_ids"]),
+                                       nb, self.cap, _ptr(b["count"]), _ptr(L["plan"]), len(plan), c0, h, w, pad, crop_thr,
+                                       float(s.relative_scale_thresh), _ptr(b["pj2d_org"]), _ptr(L["cam_full"]), _ptr(L["flags"]),
+                                       _ptr(b["sel"]), _ptr(b["count2"]), _ptr(L["base"]), _ptr(L["merged"]), L["mcap"], sp),
+           "bev_long_crops")
+        for k in self._long_fields:
+            src = L["cam_full"] if k == "cam" else b[k]
+            ck(lib.b200romp_gather_rows_at(_ptr(src), src[0].numel() * 4, _ptr(b["sel"]), _ptr(b["count2"]), _ptr(L["base"]),
+                                           self.cap, _ptr(L["m"][k]), sp), "gather_rows_at")
+
+    def _long_finish(self, h, w):
+        """bev/main.py:253-256 over all merged people, survivors gathered into the output buffers."""
+        lib, L, m, sp, ck = self.lib, self._long, self._long["m"], C.c_void_p(self.stream.cuda_stream), _lib.check
+        s, mcap = self.settings, self._long["mcap"]
+        full_thr = float(s.nms_thresh) * max(h, w, 3) / 640                # image.shape has 3 entries (main.py:255)
+        ck(lib.b200romp_bev_long_merge(_ptr(m["joints"]), _ptr(m["cam"]), _ptr(m["conf"]), mcap, _ptr(L["merged"]), h, w, full_thr,
+                                       float(s.relative_scale_thresh), _ptr(L["cam_trans"]), _ptr(L["pj2d_org"]), _ptr(L["ws"]),
+                                       _ptr(L["sel"]), _ptr(L["count_out"]), sp), "bev_long_merge")
+        for k, dst in L["o"].items():
+            src = L[k] if k in ("cam_trans", "pj2d_org") else m[k]
+            ck(lib.b200romp_gather_rows(_ptr(src), src[0].numel() * 4, _ptr(L["sel"]), _ptr(L["count_out"]), mcap, _ptr(dst), sp),
+               "gather_rows")
+        self.count_host[0:1].copy_(L["count_out"], non_blocking=True)
+
+    def _long_collect(self, to_numpy=True):
+        self.stream.synchronize()                                           # the one host synchronisation of a wide image
+        n = int(self.count_host[0])
+        if n == 0:
+            return None
+        o = self._long["o"]
+        out = {"smpl_thetas": o["thetas"][:n], "smpl_betas": o["betas"][:n], "cam": o["cam"][:n], "cam_trans": o["cam_trans"][:n],
+               "params_pred": o["params_pred"][:n], "center_confs": o["conf"][:n],
+               "pred_batch_ids": torch.zeros(n, dtype=torch.int64, device=self.tdevice), "verts": o["verts"][:n],
+               "joints": o["joints"][:n], "pj2d_org": o["pj2d_org"][:n]}
+        if to_numpy:
+            out = {k: v.cpu().numpy() for k, v in out.items()}
+        return out
+
     @torch.no_grad()
     def forward(self, image, signal_ID=0, **kwargs):
-        """image: HxWx3 uint8 BGR.  bev/main.py:139-156 (normal images; the >=2:1 panoramic tiling is out of scope)."""
+        """image: HxWx3 uint8 BGR.  bev/main.py:139-156; with ``crowd`` (the default) an image of aspect ratio >= 2 goes
+        through ``process_long_image``."""
         if image.shape[1] / image.shape[0] >= 2 and self.settings.crowd:
-            raise NotImplementedError("long-image sliding-window processing (bev/split2process.py) is out of scope")
+            return self.process_long_image(image, show_patch_results=getattr(self.settings, "show_patch_results", False))
         inp, pad = img_preprocess(image)
         out = self.forward_batch(torch.from_numpy(inp), offsets=pad, img_max_side=float(max(image.shape[:2])))
         if out is None:

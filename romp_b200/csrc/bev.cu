@@ -386,40 +386,47 @@ __global__ void __launch_bounds__(128) bev_project_kernel(const float* __restric
   pj2d_org[((size_t)n * 71 + j) * 2 + 1] = (v + 1.f) * size / 2.f - top;
 }
 
-// one CTA per frame: both reference post-filters on that frame's (<= 64) persons, then flags for the survivors
+// one CTA per frame: both reference post-filters on that frame's (<= 64) persons, then flags for the survivors.
+// conf == NULL: the duplicate with the smaller scale goes (bev/post_parser.py:195); else the one with the lower centre
+// confidence (conf_based, :191-193, crowd mode).  valid == NULL: every person of the frame takes part; else only those with
+// valid[n] != 0 (crowd mode's boundary exclusion ran first), the others keep their 0 flag.
 __global__ void __launch_bounds__(256) bev_postfilter_kernel(const float* __restrict__ pj2d_org, const float* __restrict__ cam,
                                                              const float* __restrict__ cam_trans, const long long* __restrict__ batch_ids,
                                                              const int* __restrict__ d_count, float nms_thr_px, float rel_scale_thresh,
-                                                             int* __restrict__ keep) {
-  __shared__ int s_start, s_n;
-  __shared__ int s_removed[kMaxP], s_kept[kMaxP], s_nk;
+                                                             const float* __restrict__ conf, float scale_thresh,
+                                                             const int* __restrict__ valid, int* __restrict__ keep) {
+  __shared__ int s_n;
+  __shared__ int s_idx[kMaxP], s_removed[kMaxP], s_kept[kMaxP], s_nk;
   __shared__ float s_mean[kMaxP];
   const int b = blockIdx.x, tid = threadIdx.x;
   const int N = *d_count;
   if (tid == 0) {
     int s = 0;
     while (s < N && batch_ids[s] < b) ++s;
-    int e = s;
-    while (e < N && batch_ids[e] == b) ++e;
-    s_start = s; s_n = min(e - s, kMaxP);
+    int k = 0;
+    for (int e = s; e < N && batch_ids[e] == b && k < kMaxP; ++e)
+      if (!valid || valid[e]) s_idx[k++] = e;
+    s_n = k;
   }
   if (tid < kMaxP) s_removed[tid] = 0;
   __syncthreads();
-  const int st = s_start, nf = s_n;
+  const int nf = s_n;
   if (nf == 0) return;
   if (nf > 1) {       // suppressing_redundant_prediction_via_projection, bev/post_parser.py:167-198
     for (int pr = tid; pr < nf * nf; pr += 256) {
       const int i = pr / nf, j = pr % nf;
       if (i >= j) continue;
-      const float* a = pj2d_org + (size_t)(st + i) * 142;
-      const float* c = pj2d_org + (size_t)(st + j) * 142;
+      const int ni = s_idx[i], nj = s_idx[j];
+      const float* a = pj2d_org + (size_t)ni * 142;
+      const float* c = pj2d_org + (size_t)nj * 142;
       float sum = 0.f;
       for (int k = 0; k < 71; ++k) {
         const float dx = a[2 * k] - c[2 * k], dy = a[2 * k + 1] - c[2 * k + 1];
         sum += sqrtf(dx * dx + dy * dy);
       }
-      const float si = cam[(st + i) * 3] * 2.f, sj = cam[(st + j) * 3] * 2.f;
-      if (sum / 71.f / fmaxf(si, sj) < nms_thr_px) atomicExch(&s_removed[si < sj ? i : j], 1);
+      const float si = cam[ni * 3] * 2.f, sj = cam[nj * 3] * 2.f;
+      const bool lose_i = conf ? conf[ni] < conf[nj] : si < sj;
+      if (sum / 71.f / fmaxf(si, sj) < nms_thr_px) atomicExch(&s_removed[lose_i ? i : j], 1);
     }
   }
   __syncthreads();
@@ -433,10 +440,10 @@ __global__ void __launch_bounds__(256) bev_postfilter_kernel(const float* __rest
   const int nk = s_nk;
   if (nk >= 3) {      // remove_outlier, bev/post_parser.py:200-222
     if (tid < nk) {
-      const float* ti = cam_trans + (size_t)(st + s_kept[tid]) * 3;
+      const float* ti = cam_trans + (size_t)s_idx[s_kept[tid]] * 3;
       float sum = 0.f, mn = CUDART_INF_F, mx = -CUDART_INF_F;
       for (int j = 0; j < nk; ++j) {
-        const float* tj = cam_trans + (size_t)(st + s_kept[j]) * 3;
+        const float* tj = cam_trans + (size_t)s_idx[s_kept[j]] * 3;
         const float dx = ti[0] - tj[0], dy = ti[1] - tj[1], dz = ti[2] - tj[2];
         const float d = sqrtf(dx * dx + dy * dy + dz * dz);
         sum += d; mn = fminf(mn, d); mx = fmaxf(mx, d);
@@ -448,11 +455,169 @@ __global__ void __launch_bounds__(256) bev_postfilter_kernel(const float* __rest
       float tot = 0.f;
       for (int j = 0; j < nk; ++j) tot += s_mean[j];
       const float rel = s_mean[tid] / ((tot - s_mean[tid]) / (float)(nk - 1));
-      if (rel > rel_scale_thresh && cam[(st + s_kept[tid]) * 3] < 0.25f) s_removed[s_kept[tid]] = 1;
+      if (rel > rel_scale_thresh && cam[s_idx[s_kept[tid]] * 3] < scale_thresh) s_removed[s_kept[tid]] = 1;
     }
     __syncthreads();
   }
-  if (tid < nf) keep[st + tid] = s_removed[tid] ? 0 : 1;
+  if (tid < nf) keep[s_idx[tid]] = s_removed[tid] ? 0 : 1;
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// Crowd mode (BEV.process_long_image, bev/main.py:184-258).  Crop c of the plan covers padded columns [plan[2c], plan[2c+1]);
+// drop_boundary_ratio r_c = (right_c - left_{c+1}) / h / 2 (:213-214, :223-224), evaluated in fp64 like numpy and rounded
+// to fp32 for the comparison like torch against a Python scalar.
+__device__ __forceinline__ double drop_ratio(const int* plan, int c, int h) {
+  return (double)(plan[2 * c + 1] - plan[2 * c + 2]) / (double)h / 2.0;
+}
+
+// exclude_boudary_subjects (split2process.py:41-46, tolerance 0): every crop but the last drops cam_x > 1 - r_c
+// (bev/main.py:209-215); crop c+1 drops cam_x < r_c - 1 for c in 1..S-2 (:221-226), so crop 1 is never tested on its left.
+__global__ void __launch_bounds__(256) bev_long_boundary_kernel(const float* __restrict__ cam, const long long* __restrict__ batch_ids,
+                                                                const int* __restrict__ d_count, const int* __restrict__ plan,
+                                                                int n_crops, int first_crop, int h, int* __restrict__ valid) {
+  const int n = blockIdx.x * 256 + threadIdx.x;
+  if (n >= *d_count) return;
+  const int c = (int)batch_ids[n] + first_crop;
+  const float x = cam[n * 3 + 2];
+  bool drop = false;
+  if (c != n_crops - 1) drop = x > (float)(1.0 - drop_ratio(plan, c, h) + 0.0);
+  if (c >= 2) drop = drop || x < (float)(drop_ratio(plan, c - 1, h) - 1.0 - 0.0);
+  valid[n] = drop ? 0 : 1;
+}
+
+// convert_crop_cam_params2full_image (split2process.py:48-58) with the crop box shifted by -pad (bev/main.py:247): all three
+// components times max(crop w, crop h) / max(h, w), then cam_x += mean(left, right) / (w/2) - 1.  Both factors are fp64
+// numpy scalars that torch rounds to fp32; no FMA contraction, like torch's two separate ops.
+__global__ void __launch_bounds__(256) bev_long_cam_kernel(const float* __restrict__ cam, const long long* __restrict__ batch_ids,
+                                                           const int* __restrict__ d_count, const int* __restrict__ plan, int first_crop,
+                                                           int pad, int h, int w, float* __restrict__ cam_full) {
+  const int n = blockIdx.x * 256 + threadIdx.x;
+  if (n >= *d_count) return;
+  const int c = (int)batch_ids[n] + first_crop;
+  const int l = plan[2 * c] - pad, r = plan[2 * c + 1] - pad;
+  const float sc = (float)((double)max(r - l, h) / (double)max(h, w));
+  const float dx = (float)((double)(l + r) / 2.0 / ((double)w / 2.0) - 1.0);
+  cam_full[n * 3 + 0] = __fmul_rn(cam[n * 3 + 0], sc);
+  cam_full[n * 3 + 1] = __fmul_rn(cam[n * 3 + 1], sc);
+  cam_full[n * 3 + 2] = __fadd_rn(__fmul_rn(cam[n * 3 + 2], sc), dx);
+}
+
+// survivors of this chunk of crops, in order, appended to the merged buffers: sel / *d_count_sel as bev_compact_kernel,
+// *d_base = first merged row of this chunk, *d_merged advanced (clamped to merged_capacity).
+__global__ void bev_long_append_kernel(const int* __restrict__ keep, const int* __restrict__ d_count, int merged_capacity,
+                                       int* __restrict__ sel, int* __restrict__ d_count_sel, int* __restrict__ d_base,
+                                       int* __restrict__ d_merged) {
+  if (threadIdx.x != 0 || blockIdx.x != 0) return;
+  const int N = *d_count, base = *d_merged;
+  int k = 0;
+  for (int i = 0; i < N && base + k < merged_capacity; ++i)
+    if (keep[i]) sel[k++] = i;
+  *d_count_sel = k;
+  *d_base = base;
+  *d_merged = base + k;
+}
+
+// denormalize_cam_params_to_trans (bev/post_parser.py:114-128), as in bev_unpack_kernel
+__global__ void __launch_bounds__(256) bev_cam_trans_kernel(const float* __restrict__ cam, const int* __restrict__ d_count,
+                                                            float* __restrict__ cam_trans) {
+  const int n = blockIdx.x * 256 + threadIdx.x;
+  if (n >= *d_count) return;
+  const float depth = 1.f / (cam[n * 3] * kTanFov + 1e-3f);
+  cam_trans[n * 3 + 0] = cam[n * 3 + 2] * depth * kTanFov;
+  cam_trans[n * 3 + 1] = cam[n * 3 + 1] * depth * kTanFov;
+  cam_trans[n * 3 + 2] = depth;
+}
+
+// global suppressing_redundant_prediction_via_projection(conf_based=True) (bev/main.py:255) over all merged people: one
+// thread per pair (i < j), block row i staged in shared memory; every pair is judged at once, the lower confidence goes.
+constexpr int kPairThreads = 128;
+__global__ void __launch_bounds__(kPairThreads) bev_long_pairs_kernel(const float* __restrict__ pj2d_org, const float* __restrict__ cam,
+                                                                      const float* __restrict__ conf, const int* __restrict__ d_count,
+                                                                      float nms_thr_px, int* __restrict__ removed) {
+  __shared__ float s_a[142];
+  const int i = blockIdx.y, N = *d_count;
+  if (i >= N || (int)(blockIdx.x * kPairThreads + kPairThreads - 1) <= i) return;
+  for (int k = threadIdx.x; k < 142; k += kPairThreads) s_a[k] = pj2d_org[(size_t)i * 142 + k];
+  __syncthreads();
+  const int j = blockIdx.x * kPairThreads + threadIdx.x;
+  if (j <= i || j >= N) return;
+  const float* c = pj2d_org + (size_t)j * 142;
+  float sum = 0.f;
+  for (int k = 0; k < 71; ++k) {
+    const float dx = s_a[2 * k] - c[2 * k], dy = s_a[2 * k + 1] - c[2 * k + 1];
+    sum += sqrtf(dx * dx + dy * dy);
+  }
+  const float si = cam[i * 3] * 2.f, sj = cam[j * 3] * 2.f;
+  if (sum / 71.f / fmaxf(si, sj) < nms_thr_px) atomicExch(&removed[conf[i] < conf[j] ? i : j], 1);
+}
+
+__global__ void bev_long_kept_kernel(const int* __restrict__ removed, const int* __restrict__ d_count, int* __restrict__ kept,
+                                     int* __restrict__ d_nk) {
+  if (threadIdx.x != 0 || blockIdx.x != 0) return;
+  const int N = *d_count;
+  int k = 0;
+  for (int i = 0; i < N; ++i)
+    if (!removed[i]) kept[k++] = i;
+  *d_nk = k;
+}
+
+// remove_outlier row statistic (bev/post_parser.py:206-210) of kept person r: mean of its sorted distance row without
+// the first and last entry = (sum - min - max) / (nk - 2)
+__global__ void __launch_bounds__(256) bev_long_rowmean_kernel(const float* __restrict__ cam_trans, const int* __restrict__ kept,
+                                                               const int* __restrict__ d_nk, float* __restrict__ mean_dist) {
+  __shared__ float s_sum[256], s_mn[256], s_mx[256];
+  const int r = blockIdx.x, nk = *d_nk, tid = threadIdx.x;
+  if (nk < 3 || r >= nk) return;
+  const float* ti = cam_trans + (size_t)kept[r] * 3;
+  float sum = 0.f, mn = CUDART_INF_F, mx = -CUDART_INF_F;
+  for (int j = tid; j < nk; j += 256) {
+    const float* tj = cam_trans + (size_t)kept[j] * 3;
+    const float dx = ti[0] - tj[0], dy = ti[1] - tj[1], dz = ti[2] - tj[2];
+    const float d = sqrtf(dx * dx + dy * dy + dz * dz);
+    sum += d; mn = fminf(mn, d); mx = fmaxf(mx, d);
+  }
+  s_sum[tid] = sum; s_mn[tid] = mn; s_mx[tid] = mx;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if (tid < o) {
+      s_sum[tid] += s_sum[tid + o]; s_mn[tid] = fminf(s_mn[tid], s_mn[tid + o]); s_mx[tid] = fmaxf(s_mx[tid], s_mx[tid + o]);
+    }
+    __syncthreads();
+  }
+  if (tid == 0) mean_dist[r] = (s_sum[0] - s_mn[0] - s_mx[0]) / (float)(nk - 2);
+}
+
+// remove_outlier flags (bev/post_parser.py:212-221) over the kept people, then the survivors in order -> sel / *d_count_out
+__global__ void __launch_bounds__(1024) bev_long_outlier_kernel(const float* __restrict__ cam, const int* __restrict__ kept,
+                                                                const int* __restrict__ d_nk, const float* __restrict__ mean_dist,
+                                                                float rel_scale_thresh, float scale_thresh, int* __restrict__ removed,
+                                                                const int* __restrict__ d_count, int* __restrict__ sel,
+                                                                int* __restrict__ d_count_out) {
+  __shared__ float s_red[1024];
+  const int nk = *d_nk, tid = threadIdx.x;
+  if (nk >= 3) {
+    float t = 0.f;
+    for (int r = tid; r < nk; r += 1024) t += mean_dist[r];
+    s_red[tid] = t;
+    __syncthreads();
+    for (int o = 512; o > 0; o >>= 1) {
+      if (tid < o) s_red[tid] += s_red[tid + o];
+      __syncthreads();
+    }
+    const float tot = s_red[0];
+    for (int r = tid; r < nk; r += 1024) {
+      const float rel = mean_dist[r] / ((tot - mean_dist[r]) / (float)(nk - 1));
+      if (rel > rel_scale_thresh && cam[kept[r] * 3] < scale_thresh) removed[kept[r]] = 1;
+    }
+    __syncthreads();
+  }
+  if (tid == 0) {
+    const int N = *d_count;
+    int k = 0;
+    for (int i = 0; i < N; ++i)
+      if (!removed[i]) sel[k++] = i;
+    *d_count_out = k;
+  }
 }
 
 __global__ void bev_compact_kernel(const int* __restrict__ keep, const int* __restrict__ d_count, int* __restrict__ sel,
@@ -465,12 +630,14 @@ __global__ void bev_compact_kernel(const int* __restrict__ keep, const int* __re
   *d_count_out = k;
 }
 
+// d_base (may be NULL): device row offset into dst
 __global__ void __launch_bounds__(256) gather_rows_kernel(const uint32_t* __restrict__ src, int row_words, const int* __restrict__ sel,
-                                                          const int* __restrict__ d_count, uint32_t* __restrict__ dst) {
+                                                          const int* __restrict__ d_count, const int* __restrict__ d_base,
+                                                          uint32_t* __restrict__ dst) {
   const int i = blockIdx.x;
   if (i >= *d_count) return;
   const uint32_t* s = src + (size_t)sel[i] * row_words;
-  uint32_t* d = dst + (size_t)i * row_words;
+  uint32_t* d = dst + ((size_t)(d_base ? *d_base : 0) + i) * row_words;
   for (int k = blockIdx.y * 256 + threadIdx.x; k < row_words; k += gridDim.y * 256) d[k] = s[k];
 }
 
@@ -618,7 +785,7 @@ int b200romp_bev_post(const float* betas, const float* verts_smil, const float* 
   bev_project_kernel<<<capacity, 128, 0, stream>>>(joints, cam_trans, d_count, hh > ww ? hh : ww, left, top, pj2d_org);
   B2R_CUDA_OK(cudaMemsetAsync(keep, 0, sizeof(int) * capacity, stream));
   bev_postfilter_kernel<<<batch, 256, 0, stream>>>(pj2d_org, cam, cam_trans, batch_ids, d_count, nms_thresh * img_max_side / 640.f,
-                                                   rel_scale_thresh, keep);
+                                                   rel_scale_thresh, nullptr, 0.25f, nullptr, keep);
   bev_compact_kernel<<<1, 32, 0, stream>>>(keep, d_count, sel, d_count_out);
   B2R_CUDA_OK(cudaGetLastError());
   return B200ROMP_OK;
@@ -626,10 +793,65 @@ int b200romp_bev_post(const float* betas, const float* verts_smil, const float* 
 
 int b200romp_gather_rows(const void* src, int row_bytes, const int* sel, const int* d_count, int capacity, void* dst,
                          b200romp_stream stream) {
+  return b200romp_gather_rows_at(src, row_bytes, sel, d_count, nullptr, capacity, dst, stream);
+}
+
+int b200romp_gather_rows_at(const void* src, int row_bytes, const int* sel, const int* d_count, const int* d_base, int capacity,
+                            void* dst, b200romp_stream stream) {
   B2R_REQUIRE(src && sel && d_count && dst && row_bytes > 0 && row_bytes % 4 == 0 && capacity > 0, "gather_rows: bad arguments");
   const int words = row_bytes / 4;
   gather_rows_kernel<<<dim3(capacity, words > 4096 ? 8 : 1), 256, 0, (cudaStream_t)stream>>>(
-      reinterpret_cast<const uint32_t*>(src), words, sel, d_count, reinterpret_cast<uint32_t*>(dst));
+      reinterpret_cast<const uint32_t*>(src), words, sel, d_count, d_base, reinterpret_cast<uint32_t*>(dst));
+  B2R_CUDA_OK(cudaGetLastError());
+  return B200ROMP_OK;
+}
+
+int b200romp_bev_long_crops(const float* betas, const float* verts_smil, const float* joints_smil, float* verts, float* joints,
+                            const float* cam, const float* cam_trans, const float* conf, const long long* batch_ids, int batch,
+                            int capacity, const int* d_count, const int* plan, int n_crops, int first_crop, int h, int w, int pad,
+                            float crop_nms_thr_px, float rel_scale_thresh, float* pj2d_org, float* cam_full, int* flags, int* sel,
+                            int* d_count_sel, int* d_base, int* d_merged, int merged_capacity, b200romp_stream stream_) {
+  B2R_REQUIRE(betas && verts && joints && cam && cam_trans && conf && batch_ids && d_count && plan && pj2d_org && cam_full && flags &&
+                  sel && d_count_sel && d_base && d_merged && batch > 0 && capacity > 0 && n_crops >= 2 && first_crop >= 0 &&
+                  first_crop + batch <= n_crops && h > 0 && w > 0 && pad >= 0 && merged_capacity > 0,
+              "bev_long_crops: bad arguments");
+  cudaStream_t stream = (cudaStream_t)stream_;
+  int *valid = flags, *keep = flags + capacity;
+  const unsigned g = (unsigned)((capacity + 255) / 256);
+  if (verts_smil && joints_smil)
+    bev_merge_smil_kernel<<<dim3(capacity, 4), 256, 0, stream>>>(betas, d_count, verts_smil, joints_smil, verts, joints);
+  bev_long_boundary_kernel<<<g, 256, 0, stream>>>(cam, batch_ids, d_count, plan, n_crops, first_crop, h, valid);
+  // crop pixels: input2org_offsets [0, ch, 0, cw, ch, cw] (bev/main.py:216-217); the crop width never exceeds h
+  bev_project_kernel<<<capacity, 128, 0, stream>>>(joints, cam_trans, d_count, (float)h, 0.f, 0.f, pj2d_org);
+  B2R_CUDA_OK(cudaMemsetAsync(keep, 0, sizeof(int) * capacity, stream));
+  bev_postfilter_kernel<<<batch, 256, 0, stream>>>(pj2d_org, cam, cam_trans, batch_ids, d_count, crop_nms_thr_px, rel_scale_thresh,
+                                                   conf, 1.f, valid, keep);                   // :228-232
+  bev_long_cam_kernel<<<g, 256, 0, stream>>>(cam, batch_ids, d_count, plan, first_crop, pad, h, w, cam_full);
+  bev_long_append_kernel<<<1, 32, 0, stream>>>(keep, d_count, merged_capacity, sel, d_count_sel, d_base, d_merged);
+  B2R_CUDA_OK(cudaGetLastError());
+  return B200ROMP_OK;
+}
+
+int b200romp_bev_long_merge(const float* joints, const float* cam, const float* conf, int capacity, const int* d_count, int h, int w,
+                            float nms_thr_px, float rel_scale_thresh, float* cam_trans, float* pj2d_org, int* workspace, int* sel,
+                            int* d_count_out, b200romp_stream stream_) {
+  B2R_REQUIRE(joints && cam && conf && d_count && cam_trans && pj2d_org && workspace && sel && d_count_out && capacity > 0 && h > 0 &&
+                  w > 0, "bev_long_merge: bad arguments");
+  B2R_REQUIRE(capacity <= 65535, "bev_long_merge: capacity > 65535");
+  cudaStream_t stream = (cudaStream_t)stream_;
+  int *removed = workspace, *kept = workspace + capacity, *d_nk = workspace + 2 * capacity;
+  float* mean_dist = reinterpret_cast<float*>(workspace + 2 * capacity + 1);
+  const unsigned g = (unsigned)((capacity + 255) / 256);
+  const int side = h > w ? h : w;
+  bev_cam_trans_kernel<<<g, 256, 0, stream>>>(cam, d_count, cam_trans);                       // bev/main.py:253
+  bev_project_kernel<<<capacity, 128, 0, stream>>>(joints, cam_trans, d_count, (float)side, 0.f, (float)((w - h) / 2), pj2d_org);
+  B2R_CUDA_OK(cudaMemsetAsync(removed, 0, sizeof(int) * capacity, stream));
+  bev_long_pairs_kernel<<<dim3((capacity + kPairThreads - 1) / kPairThreads, capacity), kPairThreads, 0, stream>>>(
+      pj2d_org, cam, conf, d_count, nms_thr_px, removed);                                     // :255
+  bev_long_kept_kernel<<<1, 32, 0, stream>>>(removed, d_count, kept, d_nk);
+  bev_long_rowmean_kernel<<<capacity, 256, 0, stream>>>(cam_trans, kept, d_nk, mean_dist);     // :256
+  bev_long_outlier_kernel<<<1, 1024, 0, stream>>>(cam, kept, d_nk, mean_dist, rel_scale_thresh, 0.5f, removed, d_count, sel,
+                                                  d_count_out);
   B2R_CUDA_OK(cudaGetLastError());
   return B200ROMP_OK;
 }

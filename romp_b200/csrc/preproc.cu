@@ -35,11 +35,12 @@ __device__ __forceinline__ void cubic_taps(int d, double scale, int* s0, int (&w
   *s0 = s;
 }
 
-// thread = one output pixel (3 channels)
-__global__ void __launch_bounds__(256) preprocess_bgr_kernel(const unsigned char* __restrict__ img, int h, int w, int row_stride, int side,
-                                                             int top, int left, double scale, int S, unsigned char* __restrict__ out) {
-  const int dx = blockIdx.x * blockDim.x + threadIdx.x, dy = blockIdx.y;
-  if (dx >= S) return;
+// one output pixel (3 channels) of the resize of a zero-padded square of side `side`: the square holds a win_h x win_w window
+// at (top, left) whose column c is image column col0 + c (columns outside 0..w-1 are zero too).  The replicated border
+// applies to the padded square.
+__device__ __forceinline__ void resize_pixel(const unsigned char* __restrict__ img, int h, int w, int row_stride, int win_h,
+                                             int win_w, int col0, int side, int top, int left, double scale, int dx, int dy,
+                                             unsigned char* __restrict__ o) {
   int sx, sy, ax[4], ay[4];
   cubic_taps(dx, scale, &sx, ax);
   cubic_taps(dy, scale, &sy, ay);
@@ -51,8 +52,9 @@ __global__ void __launch_bounds__(256) preprocess_bgr_kernel(const unsigned char
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       const int px = min(max(sx + j - 1, 0), side - 1) - left;
-      if ((unsigned)py < (unsigned)h && (unsigned)px < (unsigned)w) {
-        const unsigned char* p = img + (size_t)py * row_stride + (size_t)px * 3;
+      const int col = col0 + px;
+      if ((unsigned)py < (unsigned)win_h && (unsigned)px < (unsigned)win_w && (unsigned)col < (unsigned)w) {
+        const unsigned char* p = img + (size_t)py * row_stride + (size_t)col * 3;
         v0 += (int)p[2] * ax[j];                                        // RGB <- BGR
         v1 += (int)p[1] * ax[j];
         v2 += (int)p[0] * ax[j];
@@ -62,7 +64,6 @@ __global__ void __launch_bounds__(256) preprocess_bgr_kernel(const unsigned char
   }
   const float sc = 1.f / (2048.f * 2048.f);
   const float b0 = __fmul_rn((float)ay[0], sc), b1 = __fmul_rn((float)ay[1], sc), b2 = __fmul_rn((float)ay[2], sc), b3 = __fmul_rn((float)ay[3], sc);
-  unsigned char* o = out + ((size_t)dy * S + dx) * 3;
 #pragma unroll
   for (int c = 0; c < 3; ++c) {
     float t = __fmul_rn((float)rows[3][c], b3);
@@ -71,6 +72,27 @@ __global__ void __launch_bounds__(256) preprocess_bgr_kernel(const unsigned char
     t = __fadd_rn(__fmul_rn((float)rows[0][c], b0), t);
     o[c] = (unsigned char)min(max(__float2int_rn(t), 0), 255);
   }
+}
+
+// thread = one output pixel (3 channels)
+__global__ void __launch_bounds__(256) preprocess_bgr_kernel(const unsigned char* __restrict__ img, int h, int w, int row_stride, int side,
+                                                             int top, int left, double scale, int S, unsigned char* __restrict__ out) {
+  const int dx = blockIdx.x * blockDim.x + threadIdx.x, dy = blockIdx.y;
+  if (dx >= S) return;
+  resize_pixel(img, h, w, row_stride, h, w, 0, side, top, left, scale, dx, dy, out + ((size_t)dy * S + dx) * 3);
+}
+
+// crowd mode: blockIdx.z = crop.  Crop c covers rows 0..h-1 and columns plan[c] = [l, r) of the image padded by `pad` zero
+// columns on each side (split2process.py:6-39); each crop is img_preprocess'ed like a whole image (utils.py:16-30).
+__global__ void __launch_bounds__(256) preprocess_crops_kernel(const unsigned char* __restrict__ img, int h, int w, int row_stride,
+                                                               int pad, const int* __restrict__ plan, int first_crop, int S,
+                                                               unsigned char* __restrict__ out) {
+  const int dx = blockIdx.x * blockDim.x + threadIdx.x, dy = blockIdx.y, c = blockIdx.z;
+  if (dx >= S) return;
+  const int l = plan[2 * (first_crop + c)], r = plan[2 * (first_crop + c) + 1];
+  const int cw = r - l, side = h > cw ? h : cw;
+  resize_pixel(img, h, w, row_stride, h, cw, l - pad, side, (side - h) / 2, (side - cw) / 2, (double)side / (double)S, dx, dy,
+               out + (((size_t)c * S + dy) * S + dx) * 3);
 }
 
 }  // namespace b200romp
@@ -89,6 +111,18 @@ extern "C" int b200romp_preprocess_bgr(const unsigned char* img_bgr, int h, int 
   dim3 grid((out_size + 255) / 256, out_size);
   preprocess_bgr_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(img_bgr, h, w, row_stride_bytes, side, top, left, (double)side / (double)out_size,
                                                                out_size, out_rgb);
+  B2R_CUDA_OK(cudaGetLastError());
+  return B200ROMP_OK;
+}
+
+extern "C" int b200romp_preprocess_crops_bgr(const unsigned char* img_bgr, int h, int w, int row_stride_bytes, int pad,
+                                             const int* plan, int first_crop, int n_crops, int out_size, unsigned char* out_rgb,
+                                             b200romp_stream stream) {
+  B2R_REQUIRE(img_bgr && plan && out_rgb && h > 0 && w > 0 && row_stride_bytes >= 3 * w && pad >= 0 && first_crop >= 0 &&
+                  n_crops > 0 && n_crops <= 65535 && out_size > 0, "preprocess_crops_bgr: bad arguments");
+  dim3 grid((out_size + 255) / 256, out_size, n_crops);
+  preprocess_crops_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(img_bgr, h, w, row_stride_bytes, pad, plan, first_crop, out_size,
+                                                                  out_rgb);
   B2R_CUDA_OK(cudaGetLastError());
   return B200ROMP_OK;
 }

@@ -451,3 +451,36 @@ def resnet50_state_dict(seed: int = 0, gain: float = 0.8):
         elif kind == "bn_n":
             sd[name] = np.array(1, dtype=np.int64)
     return sd
+
+
+def synthetic_wide_image(h: int, w: int, seed: int = 0):
+    """HxWx3 uint8 BGR image of any size with the texture of ``synthetic_frames`` (8-pixel blocks + noise): the input of
+    BEV's crowd mode (w/h >= 2, bev/main.py:140-141)."""
+    rng = np.random.RandomState(seed + 1299709)
+    base = rng.randint(0, 256, size=(h // 8 + 1, w // 8 + 1, 3)).astype(np.float32)
+    up = np.repeat(np.repeat(base, 8, axis=0), 8, axis=1)[:h, :w]
+    noise = rng.randint(-32, 33, size=(h, w, 3)).astype(np.float32)
+    return np.clip(up + noise, 0, 255).astype(np.uint8)
+
+
+def bev_planted_crops(n_crops: int, cells, seed: int = 0):
+    """Per-crop 3-D centre maps [n_crops,64,128,128] for crowd mode: a uniform background in [0, 0.05) (below every BEV
+    centre threshold) plus the caller's cells ``(crop, z, y, x, value)``.  Cells of one crop should be >= 3 voxels apart
+    in some axis so that the 5x5x5 max-pool NMS (bev/post_parser.py:44-66) keeps each of them."""
+    rs = np.random.RandomState(seed + 49979687)
+    vol = rs.uniform(0, 0.05, size=(n_crops, 64, 128, 128)).astype(np.float32)
+    for c, z, y, x, v in cells:
+        vol[int(c), int(z), int(y), int(x)] = np.float32(v)
+    return vol
+
+
+def bev_crowd_state_dict(seed: int = 0, beta10_shift: float = 0.6735):
+    """Synthetic BEV weights of the crowd-mode tests and bench: ``bev_damp_cam_offsets`` (planted cells give
+    cam ~ coordmap_3d[z, y, x]) plus a shift of the output bias of betas[10] (transformer.6 row 142, bev/model.py:116) so
+    that some planted people are babies (betas[10] > 0.8 selects SMIL, bev/post_parser.py:260-268); the default shift
+    puts the threshold in the widest gap of the crowd-mode fixture's values."""
+    out = bev_damp_cam_offsets(bev_state_dict(seed))
+    b = np.array(out["transformer.6.bias"], np.float32, copy=True)
+    b[142] += np.float32(beta10_shift)
+    out["transformer.6.bias"] = b
+    return out
